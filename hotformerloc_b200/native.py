@@ -122,6 +122,10 @@ SIGNATURES = {
     'hfl_knn_workspace_bytes': (C.c_int64, [_i32, _i32, _i32]),
     'hfl_knn_topk_ws': (C.c_int, [_p, _i32, _p, _i32, _i32, _i32, _i32, _p, _p, _p, _i64, _p]),
     'hfl_topk_merge': (C.c_int, [_p, _p, _i32, _i32, _i32, _p, _p, _p]),
+    'hfl_dwconv': (C.c_int, [_p, _p, _i32, _p, _i64, _i64, _i32, _i32, _p, _p]),
+    'hfl_dwconv_inverse': (C.c_int, [_p, _i32, _i64, _i64, _i32, _p, _p]),
+    'hfl_dwconv_wgrad_workspace_bytes': (C.c_int64, [_i64, _i32, _i32]),
+    'hfl_dwconv_wgrad': (C.c_int, [_p, _p, _p, _i32, _i64, _i64, _i32, _i32, _p, _p, _i64, _p]),
 }
 
 

@@ -20,7 +20,14 @@ import torch
 from . import native as N
 
 BATCH_SHIFT = 48
-LUT_KERNEL = {'222': [13, 14, 16, 17, 22, 23, 25, 26], '333': list(range(27))}
+LUT_KERNEL = {                       # ocnn's kernel shapes -> columns of the 27-neighbour table
+    '222': [13, 14, 16, 17, 22, 23, 25, 26],
+    '311': [4, 13, 22], '131': [10, 13, 16], '113': [12, 13, 14],
+    '331': [1, 4, 7, 10, 13, 16, 19, 22, 25],
+    '313': [3, 4, 5, 12, 13, 14, 21, 22, 23],
+    '133': [9, 10, 11, 12, 13, 14, 15, 16, 17],
+    '333': list(range(27)),
+}
 
 
 class Points:

@@ -230,6 +230,36 @@ int hfl_prepare_clouds(const float* in, const int32_t* off_in, int32_t B, int64_
                        int32_t zero_mean, float scale_factor, float norm_range, int32_t cyl, float* tmp,
                        int32_t* cnt, float* out, int32_t* off_out, int32_t* total_out, void* stream);
 
+/* ------------------------------------------------------------------------
+ * Octree depth-wise convolution with backward, fp32 (the reference's `dwconv.core`,
+ * libs/dwconv/csrc/pybind.cpp:10-14; training-side, not called by the embedding path)
+ * neigh: [rows, K] neighbour table, int64 (neigh_i64 != 0, the reference layout) or int32,
+ * 1 <= K <= 27; an entry outside [0, n_in) (or [0, n_data)) is an empty tap.
+ * ------------------------------------------------------------------------ */
+
+/* out[i,c] = sum_k w[k,c] * data[neigh[i,k],c] over the non-empty taps; data [n_in, C], w [K, C]
+ * ((K,1,C) in the reference), out [n_out, C].  Each element is accumulated from 0.f in ascending
+ * k with fmaf, the order of the reference kernel.  With the inverse table (hfl_dwconv_inverse) in
+ * place of neigh and the output gradient in place of data it is the input gradient.
+ * Replaces dwconv_forward_backward (libs/dwconv/csrc/dwconv.cu:99-113). */
+int hfl_dwconv(const float* data, const void* neigh, int32_t neigh_i64, const float* w, int64_t n_out,
+               int64_t n_in, int32_t K, int32_t C, float* out, void* stream);
+
+/* ineigh_out [n_data, K], same dtype as neigh: ineigh[neigh[i,k], k] = i, -1 where no row points.
+ * A well-formed stride-1 octree table hits each (j,k) at most once; if several rows hit one (j,k)
+ * the entry is the largest such i (deterministic, where the reference's scatter races).
+ * Replaces inverse_neigh (libs/dwconv/csrc/dwconv.cu:74-85, :87). */
+int hfl_dwconv_inverse(const void* neigh, int32_t neigh_i64, int64_t n_rows, int64_t n_data, int32_t K,
+                       void* ineigh_out, void* stream);
+
+/* dw[k,c] = sum_i grad[i,c] * data[neigh[i,k],c]; grad [n, C], neigh [n, K], dw [K, C].  Fixed-order
+ * sums without float atomics over a row partition that depends on (n, K, C) only: bit-identical
+ * across runs and GPUs.  ws: hfl_dwconv_wgrad_workspace_bytes(n, K, C) bytes, 16-byte aligned.
+ * Replaces dwconv_weight_backward (libs/dwconv/csrc/dwconv.cu:45-72, :115). */
+int64_t hfl_dwconv_wgrad_workspace_bytes(int64_t n, int32_t K, int32_t C);
+int hfl_dwconv_wgrad(const float* grad, const float* data, const void* neigh, int32_t neigh_i64, int64_t n,
+                     int64_t n_in, int32_t K, int32_t C, float* dw, void* ws, int64_t ws_bytes, void* stream);
+
 /* Exact L2 top-k (eval/pnv_evaluate.py:200-225, 245) on one database shard, and the
  * merge of all-gathered partial lists. */
 int hfl_knn_topk(const float* q, int32_t nq, const float* db, int32_t ndb, int32_t dim, int32_t k,
