@@ -444,6 +444,87 @@ __global__ void k_counts(CountArgs a, int D, int F, int B, int32_t* __restrict__
 }
 
 // ---------------------------------------------------------------------------
+// import of an ocnn octree (all-node keys / children per depth -> the tables above)
+// ---------------------------------------------------------------------------
+// pass 1: non-empty nodes (children >= 0) per tile; pass 2 is k_uniq_scan
+__global__ void __launch_bounds__(SC_THREADS)
+k_import_count(const int32_t* __restrict__ ch, int64_t n, uint32_t* __restrict__ bsum) {
+  __shared__ uint32_t wsum[33];
+  const int64_t i0 = (int64_t)blockIdx.x * SC_TILE + (int64_t)threadIdx.x * SC_ITEMS;
+  uint32_t t = 0;
+#pragma unroll
+  for (int j = 0; j < SC_ITEMS; ++j)
+    if (i0 + j < n) t += ch[i0 + j] >= 0;
+  uint32_t total;
+  block_excl_scan_512(t, wsum, total);
+  if (threadIdx.x == 0) bsum[blockIdx.x] = total;
+}
+
+// pass 3, depth d: all-node i with children value c.  The compact key of node i follows from its
+// position alone (d <= F: i; d > F: the parent's compact key << 3 | i & 7), so nkey never holds an
+// input value; the input key is only compared with it (invariant K).  Entries are scattered by
+// their in-order rank r, never by c: c must equal r (invariant C) and a rank >= nn is dropped, so
+// every written index is in range whatever the input.  children_out keeps c only where it is that
+// rank, otherwise -1, and ranks the input leaves unfilled get node 0: the neighbour kernels index
+// through these tables before the host has seen the status.
+__global__ void __launch_bounds__(SC_THREADS)
+k_import_level(const int32_t* __restrict__ ch, const int64_t* __restrict__ keys, int64_t n,
+               int64_t nn, int d, int F, const uint64_t* __restrict__ pkey,
+               const uint32_t* __restrict__ bsum, const int32_t* __restrict__ total_ptr,
+               uint64_t* __restrict__ nkey, int32_t* __restrict__ nidx,
+               int32_t* __restrict__ children_out, int32_t* __restrict__ nn_out,
+               int32_t* __restrict__ status) {
+  __shared__ uint32_t wsum[33];
+  const int64_t i0 = (int64_t)blockIdx.x * SC_TILE + (int64_t)threadIdx.x * SC_ITEMS;
+  int32_t c[SC_ITEMS];
+  uint32_t t = 0;
+#pragma unroll
+  for (int j = 0; j < SC_ITEMS; ++j) {
+    c[j] = (i0 + j < n) ? ch[i0 + j] : -1;
+    t += c[j] >= 0;
+  }
+  uint32_t tot;
+  uint32_t r = block_excl_scan_512(t, wsum, tot) + bsum[blockIdx.x];
+  const uint64_t mmask = (1ull << (3 * d)) - 1;
+  bool bad_c = false, bad_k = false;
+#pragma unroll
+  for (int j = 0; j < SC_ITEMS; ++j) {
+    const int64_t i = i0 + j;
+    if (i < n) {
+      const uint64_t ck = d <= F ? (uint64_t)i : (pkey[i >> 3] << 3) | (uint64_t)(i & 7);
+      bad_k |= (uint64_t)keys[i] != (((ck >> (3 * d)) << 48) | (ck & mmask));
+      int32_t out = -1;
+      if (c[j] >= 0) {
+        if ((int64_t)r < nn) {
+          nidx[r] = (int32_t)i;
+          nkey[r] = ck;
+          if ((uint32_t)c[j] == r) out = c[j];
+        }
+        bad_c |= out < 0;
+        ++r;
+      } else {
+        bad_c |= c[j] != -1;
+      }
+      children_out[i] = out;
+    }
+  }
+  const int64_t total = *total_ptr;
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    *nn_out = (int32_t)nn;
+    bad_c |= total != nn;
+  }
+  for (int64_t q = total + blockIdx.x * (int64_t)blockDim.x + threadIdx.x; q < nn;
+       q += (int64_t)gridDim.x * blockDim.x) {
+    nidx[q] = 0;
+    nkey[q] = 0;
+  }
+  if (bad_c || bad_k) {
+    atomicOr(status, (bad_c ? HFL_IMPORT_BAD_CHILDREN : 0) | (bad_k ? HFL_IMPORT_BAD_KEYS : 0));
+    atomicOr(status + 1, 1 << d);
+  }
+}
+
+// ---------------------------------------------------------------------------
 // neighbours
 // ---------------------------------------------------------------------------
 __device__ __forceinline__ void lut_pc(int c, int k, int& lp, int& lc) {
@@ -668,6 +749,66 @@ int hfl_octree_build(const float* points, const int32_t* pt_offsets, const hfl_o
     const int t = (D + 1) * B;
     HFL_LAUNCH((k_counts<<<(int)ceil_div(t, 256), 256, 0, st>>>(ca, D, F, B, counts)));
   }
+  return HFL_OK;
+}
+
+size_t hfl_octree_import_workspace_bytes(const hfl_ocnn_octree* in) {
+  int64_t n = 1;
+  if (in && in->depth >= 0 && in->depth <= HFL_MAX_DEPTH)
+    for (int d = 0; d <= in->depth; ++d) n = in->nnum[d] > n ? in->nnum[d] : n;
+  return align_up(4 * (ceil_div(n, SC_TILE) + 1)) + align_up(4);
+}
+
+int hfl_octree_import_check(const hfl_ocnn_octree* in) {
+  HFL_CHECK_ARG(in, "null argument");
+  const int D = in->depth, F = in->full_depth, B = in->batch;
+  HFL_CHECK_ARG(D >= 1 && D <= HFL_MAX_DEPTH && F >= 1 && F < D, "need 1 <= full_depth < depth <= 15");
+  HFL_CHECK_ARG(B >= 1 && B < 32768, "batch must be in [1, 32767]");
+  for (int d = 0; d <= D; ++d) {
+    const int64_t nn = in->nnum[d], ne = in->nnum_nempty[d];
+    HFL_CHECK_ARG(nn < (1ll << 31) && ne >= 0 && ne <= nn, "need 0 <= nnum_nempty[d] <= nnum[d] < 2^31");
+    if (d <= F) HFL_CHECK_ARG(nn == ((int64_t)B << (3 * d)), "need nnum[d] == batch * 8^d for d <= full_depth");
+    if (d < F) HFL_CHECK_ARG(ne == nn, "need nnum_nempty[d] == nnum[d] for d < full_depth");
+    if (d > F) HFL_CHECK_ARG(nn == 8 * in->nnum_nempty[d - 1], "need nnum[d] == 8 * nnum_nempty[d-1] for d > full_depth");
+  }
+  return HFL_OK;
+}
+
+int hfl_octree_import(const hfl_ocnn_octree* in, const hfl_octree* o, int32_t* status,
+                      void* workspace, size_t workspace_bytes, void* stream_) {
+  cudaStream_t st = (cudaStream_t)stream_;
+  HFL_CHECK_ARG(in && o && status && workspace, "null argument");
+  const int rc = hfl_octree_import_check(in);
+  if (rc != HFL_OK) return rc;
+  const int D = in->depth, F = in->full_depth, B = in->batch;
+  HFL_CHECK_ARG(o->depth == D && o->full_depth == F && o->batch == B, "output octree shape differs");
+  for (int d = 0; d <= D; ++d) {
+    HFL_CHECK_ARG(in->nnum[d] == 0 || (in->keys[d] && in->children[d]), "null input array");
+    HFL_CHECK_ARG(o->cap[d] >= in->nnum_nempty[d], "node capacity too small");
+    HFL_CHECK_ARG(o->nkey[d] && o->children[d] && o->nidx[d], "null node array");
+  }
+  HFL_CHECK_ARG(in->nnum_nempty[D] == 0 || in->points, "null points");
+  HFL_CHECK_ARG(o->leaf_points && o->counts, "null output");
+  const size_t ws = hfl_octree_import_workspace_bytes(in);
+  if (ws > workspace_bytes) return fail(HFL_ERR_WORKSPACE, "workspace too small%s (need %lld)", "", (long long)ws);
+  uint32_t* bsum = (uint32_t*)workspace;
+  int32_t* total = (int32_t*)((char*)workspace + ws - align_up(4));
+  const int stride = B + 2;
+
+  HFL_CUDA(cudaMemsetAsync(status, 0, 2 * sizeof(int32_t), st));
+  for (int d = 0; d <= D; ++d) {        // top down: depth d reads the compact keys of depth d-1
+    const int64_t n = in->nnum[d];
+    const int g = (int)(ceil_div(n, SC_TILE) > 0 ? ceil_div(n, SC_TILE) : 1);
+    HFL_LAUNCH((k_import_count<<<g, SC_THREADS, 0, st>>>(in->children[d], n, bsum)));
+    HFL_LAUNCH((k_uniq_scan<<<1, 1024, 0, st>>>(bsum, nullptr, n, total)));
+    HFL_LAUNCH((k_import_level<<<g, SC_THREADS, 0, st>>>(
+        in->children[d], in->keys[d], n, in->nnum_nempty[d], d, F, d > F ? o->nkey[d - 1] : nullptr,
+        bsum, total, o->nkey[d], o->nidx[d], o->children[d], o->counts + (size_t)d * stride + B, status)));
+  }
+  HFL_CUDA(cudaMemcpyAsync(o->leaf_points, in->points, 12 * in->nnum_nempty[D], cudaMemcpyDeviceToDevice, st));
+  CountArgs ca;
+  for (int d = 0; d <= HFL_MAX_DEPTH; ++d) ca.nkey[d] = d <= D ? o->nkey[d] : nullptr;
+  HFL_LAUNCH((k_counts<<<(int)ceil_div((D + 1) * B, 256), 256, 0, st>>>(ca, D, F, B, o->counts)));
   return HFL_OK;
 }
 

@@ -22,7 +22,7 @@ import torch.nn as nn
 
 from .. import native as N
 from .. import ops
-from ..octree import Octree
+from ..octree import Octree, from_ocnn
 
 
 # ----------------------------------------------------------------------------
@@ -30,6 +30,12 @@ from ..octree import Octree
 # ----------------------------------------------------------------------------
 def _trunc(t, std=0.02):
     return nn.init.trunc_normal_(t, std=std)
+
+
+def _native_octree(octree) -> Octree:
+    """The model runs on the native Octree; an ocnn octree (what the reference's callers pass) is
+    imported on the device.  Anything else raises TypeError naming the missing attributes."""
+    return octree if isinstance(octree, Octree) else from_ocnn(octree)
 
 
 class _OctConv(nn.Module):
@@ -209,9 +215,9 @@ class HOTFormer(nn.Module):
         ``(local_feat_dict {depth: (n_d, C)}, relay_token_dict {depth: (N_win_d, C)}, octree)``.
         ``data`` must be ``InputFeature('P', nempty=True)(octree)`` -- the leaf point means the first
         kernel reads straight from the octree (only input_features='P' is on the hot path): it is
-        checked for shape and otherwise not re-read."""
-        if not isinstance(octree, Octree):
-            raise TypeError('octree must be a hotformerloc_b200.octree.Octree')
+        checked for shape and otherwise not re-read.  ``octree`` may be an ocnn octree; the third
+        output is then the native Octree imported from it."""
+        octree = _native_octree(octree)
         assert depth == octree.depth, 'the backbone starts at the leaf depth of the octree'
         if data is not None:
             assert tuple(data.shape) == (octree.n(octree.depth), 3), \
@@ -739,7 +745,8 @@ class _Engine:
 
 class HOTFormerLoc(nn.Module):
     """Same constructor and ``forward(batch) -> {'global': (B, output_dim)}`` as the
-    reference (models/hotformerloc.py:18-59)."""
+    reference (models/hotformerloc.py:18-59); ``batch['octree']`` is a native Octree or an ocnn
+    octree."""
 
     def __init__(self, backbone: nn.Module, pooling: PoolingWrapper,
                  normalize_embeddings: bool = False, input_features='P'):
@@ -762,17 +769,14 @@ class HOTFormerLoc(nn.Module):
         self._engine.invalidate()
 
     def forward(self, batch):
-        octree = batch['octree']
-        if not isinstance(octree, Octree):
-            raise TypeError("batch['octree'] must be a hotformerloc_b200.octree.Octree "
-                            '(build it with hotformerloc_b200.octree.build_batch or merge_octrees)')
+        octree = _native_octree(batch['octree'])
         self._engine.normalize_embeddings = self.normalize_embeddings
         x = self._engine.forward(octree)
         assert x.dim() == 2 and x.shape[1] == self.pooling.output_dim
         return {'global': x}
 
     def forward_debug(self, batch):
-        return self._engine.forward(batch['octree'], return_intermediates=True)
+        return self._engine.forward(_native_octree(batch['octree']), return_intermediates=True)
 
     def print_info(self):
         print('Model class: HOTFormerLoc (B200-native)')

@@ -43,6 +43,21 @@ class hfl_octree(C.Structure):
     ]
 
 
+class hfl_ocnn_octree(C.Structure):
+    _fields_ = [
+        ('depth', C.c_int32), ('full_depth', C.c_int32), ('batch', C.c_int32), ('_pad', C.c_int32),
+        ('nnum', C.c_int64 * (HFL_MAX_DEPTH + 1)),
+        ('nnum_nempty', C.c_int64 * (HFL_MAX_DEPTH + 1)),
+        ('keys', C.c_void_p * (HFL_MAX_DEPTH + 1)),
+        ('children', C.c_void_p * (HFL_MAX_DEPTH + 1)),
+        ('points', C.c_void_p),
+    ]
+
+
+HFL_IMPORT_BAD_CHILDREN = 1
+HFL_IMPORT_BAD_KEYS = 2
+
+
 def sources():
     return sorted(glob.glob(os.path.join(CSRC, '*.cu')))
 
@@ -92,6 +107,9 @@ SIGNATURES = {
     'hfl_launch_count': (_i64, []),
     'hfl_octree_build_workspace_bytes': (_sz, [_i64, _i32, _i32]),
     'hfl_octree_build': (C.c_int, [_p, _p, C.POINTER(hfl_octree), _p, _sz, _p]),
+    'hfl_octree_import_check': (C.c_int, [C.POINTER(hfl_ocnn_octree)]),
+    'hfl_octree_import_workspace_bytes':(_sz, [C.POINTER(hfl_ocnn_octree)]),
+    'hfl_octree_import': (C.c_int, [C.POINTER(hfl_ocnn_octree), C.POINTER(hfl_octree), _p, _p, _sz, _p]),
     'hfl_octree_neigh': (C.c_int, [C.POINTER(hfl_octree), _i32, _p, _p, _p, _p, _p]),
     'hfl_octree_neigh_full': (C.c_int, [C.POINTER(hfl_octree), _i32, _p, _p, _p]),
     'hfl_octree_full_keys': (C.c_int, [C.POINTER(hfl_octree), _i32, _p, _p]),

@@ -99,20 +99,36 @@ class Octree:
     def _build_device(self, pts: torch.Tensor, offs: torch.Tensor, n: int,
                       want_point_leaf: bool = False, neigh: bool = True):
         L = N.lib()
-        B, D, F, dev = self.batch_size, self.depth, self.full_depth, self.device
+        B, D, F = self.batch_size, self.depth, self.full_depth
         cap = []
         for d in range(D + 1):
             full = B * 8 ** d
             cap.append(full if d <= F else min(full, n))
+        self._carve(cap, n)
+        desc = self._desc
+        desc.point_leaf = self._point_leaf.data_ptr() if want_point_leaf else None
+        ws_bytes = int(L.hfl_octree_build_workspace_bytes(n, B, D))
+        ws = _arena(ws_bytes, self.device)
+        N.check(L.hfl_octree_build(N.ptr(pts), N.ptr(offs), C.byref(desc), N.ptr(ws), ws_bytes,
+                                   N.stream()))
+        self._read_back_counts()
+        self._pts_keepalive = (pts, offs, ws)
+        if neigh:
+            self._construct_ne_all()
+
+    def _carve(self, cap: List[int], n: int, n_status: int = 0):
+        """One arena for the node arrays of row capacity cap[d] (d <= full_depth: batch*8^d), the
+        leaf means, the point -> leaf map of n points and the counts table followed by n_status
+        int32; self._desc describes it."""
+        B, D, F = self.batch_size, self.depth, self.full_depth
         al = lambda x: (x + 255) // 256 * 256
+        n_counts = (D + 1) * (B + 2) + n_status
         sz_key = [al(8 * cap[d]) for d in range(D + 1)]
         sz_idx = [al(4 * cap[d]) for d in range(D + 1)]
         sz_chl = [al(4 * (cap[d] if d <= F else 8 * cap[d - 1])) for d in range(D + 1)]
-        ws_bytes = int(L.hfl_octree_build_workspace_bytes(n, B, D))
         total = sum(sz_key) + sum(sz_idx) + sum(sz_chl) + al(12 * cap[D]) + al(4 * n) \
-            + al(4 * (D + 1) * (B + 2))
-        arena = _arena(total, dev)
-        ws = _arena(ws_bytes, dev)
+            + al(4 * n_counts)
+        arena = _arena(total, self.device)
         self._arena = arena
         base = arena.data_ptr()
         pos = 0
@@ -134,26 +150,22 @@ class Octree:
             desc.nkey[d], desc.nidx[d], desc.children[d] = k.data_ptr(), i.data_ptr(), c.data_ptr()
         self._leaf_points = take(al(12 * cap[D]), torch.float32, 3 * cap[D])
         self._point_leaf = take(al(4 * n), torch.int32, n)
-        self._counts_dev = take(al(4 * (D + 1) * (B + 2)), torch.int32, (D + 1) * (B + 2))
+        self._counts_dev = take(al(4 * n_counts), torch.int32, n_counts)
         desc.leaf_points = self._leaf_points.data_ptr()
-        desc.point_leaf = self._point_leaf.data_ptr() if want_point_leaf else None
         desc.counts = self._counts_dev.data_ptr()
         self._desc, self._cap, self._n_points = desc, cap, n
-        N.check(L.hfl_octree_build(N.ptr(pts), N.ptr(offs), C.byref(desc), N.ptr(ws), ws_bytes,
-                                   N.stream()))
-        # counts -> host (the only D2H of the build; shapes of every later tensor).  The pinned slot is
-        # shared and rotates: finalize() re-reads from the device if it was handed out again meanwhile.
-        self._counts_host = N.pinned_d2h.take(4 * (D + 1) * (B + 2)).view(torch.int32).view(D + 1, B + 2)
+
+    def _read_back_counts(self):
+        # counts (+ import status) -> host: the only D2H of the build; shapes of every later tensor.  The
+        # pinned slot is shared and rotates: finalize() re-reads from the device if it was handed out again.
+        self._counts_host = N.pinned_d2h.take(4 * self._counts_dev.numel()).view(torch.int32)
         self._counts_slot = N.pinned_d2h.ticket()
-        self._counts_host.copy_(self._counts_dev.view(D + 1, B + 2), non_blocking=True)
+        self._counts_host.copy_(self._counts_dev, non_blocking=True)
         N.pinned_d2h.mark()
         self._ready = torch.cuda.Event()
         self._ready.record()
-        self._pts_keepalive = (pts, offs, ws)
         self._built = True
         self._finalized = False
-        if neigh:
-            self._construct_ne_all()
 
     def _construct_ne_all(self):
         """Non-empty 27-neighbour tables for every depth >= full_depth, capacity
@@ -184,11 +196,14 @@ class Octree:
         if self._finalized:
             return self
         self._ready.synchronize()
-        B = self.batch_size
+        B, D = self.batch_size, self.depth
         if N.pinned_d2h.valid(self._counts_slot):
             c = self._counts_host.to(torch.int64)    # copies out of the pinned staging slot
         else:                                        # the slot served a later build: read the device copy
-            c = self._counts_dev.view(self.depth + 1, B + 2).cpu().to(torch.int64)
+            c = self._counts_dev.cpu().to(torch.int64)
+        status, c = c[(D + 1) * (B + 2):], c[:(D + 1) * (B + 2)].view(D + 1, B + 2)
+        if status.numel():
+            _check_import(status, c[:, :B], self._ocnn_batch_nnum_nempty)
         self.batch_nnum_nempty = c[:, :B].clone()
         self.nnum_nempty = c[:, B].clone()
         self.nnum = c[:, B + 1].clone()
@@ -337,6 +352,110 @@ def build_batch_device(points: torch.Tensor, offsets: torch.Tensor, depth: int,
     o._src = ('device', points, offsets)
     o._build_device(points, offsets, int(points.shape[0]), False, neigh)
     return o
+
+
+OCNN_ATTRS = ('depth', 'full_depth', 'batch_size', 'keys', 'children', 'points', 'nnum', 'nnum_nempty',
+              'batch_nnum_nempty')
+
+
+def from_ocnn(octree) -> Octree:
+    """The native Octree of an ocnn octree (the merged batch octree the reference's collate_batch +
+    to_device build, eval/pnv_evaluate.py:122-126, 173-176), converted and checked on the device.
+
+    Reads ``depth, full_depth, batch_size, nnum, nnum_nempty, batch_nnum_nempty`` and the per-depth
+    ``keys`` (int64), ``children`` (int32) and ``points[depth]`` (fp32, leaf means in octree units).
+    Tensors already on the GPU are used in place; CPU tensors go up in one pinned host-to-device
+    copy.  ocnn's ``neighs``, ``features`` and ``normals`` are not read: the neighbour tables are
+    rebuilt.  Count relations, lengths and dtypes are checked on the host before anything reaches the
+    device (HflError); the structure of keys / children is checked by the import kernel, and
+    ``finalize()`` (called by every consumer) raises HflError naming the violated invariant."""
+    missing = [a for a in OCNN_ATTRS if not hasattr(octree, a)]
+    if missing:
+        raise TypeError(f'expected a hotformerloc_b200.octree.Octree or an ocnn octree; '
+                        f'{type(octree).__name__} has no {", ".join(missing)}')
+    L = N.lib()
+    D, F, B = int(octree.depth), int(octree.full_depth), int(octree.batch_size)
+    if not 1 <= D <= N.HFL_MAX_DEPTH:
+        raise N.HflError(f'depth {D} is outside [1, {N.HFL_MAX_DEPTH}]')
+    nnum = [int(x) for x in torch.as_tensor(octree.nnum).reshape(-1).tolist()]
+    nnum_nempty = [int(x) for x in torch.as_tensor(octree.nnum_nempty).reshape(-1).tolist()]
+    if len(nnum) != D + 1 or len(nnum_nempty) != D + 1:
+        raise N.HflError(f'nnum and nnum_nempty need depth + 1 = {D + 1} entries')
+    desc = N.hfl_ocnn_octree()
+    desc.depth, desc.full_depth, desc.batch = D, F, B
+    for d in range(D + 1):
+        desc.nnum[d], desc.nnum_nempty[d] = nnum[d], nnum_nempty[d]
+    N.check(L.hfl_octree_import_check(C.byref(desc)))
+
+    def tensor(t, dtype, shape, name):
+        if not isinstance(t, torch.Tensor) or t.dtype != dtype or tuple(t.shape) != shape:
+            got = (t.dtype, tuple(t.shape)) if isinstance(t, torch.Tensor) else type(t).__name__
+            raise N.HflError(f'{name} must be a {dtype} tensor of shape {shape}, got {got}')
+        return t.contiguous()
+    arrays = [tensor(octree.keys[d], torch.int64, (nnum[d],), f'keys[{d}]') for d in range(D + 1)]
+    arrays += [tensor(octree.children[d], torch.int32, (nnum[d],), f'children[{d}]') for d in range(D + 1)]
+    arrays.append(tensor(octree.points[D], torch.float32, (nnum_nempty[D], 3), f'points[{D}]'))
+    bnn = torch.as_tensor(octree.batch_nnum_nempty).cpu()
+    if tuple(bnn.shape) != (D + 1, B):
+        raise N.HflError(f'batch_nnum_nempty must have shape {(D + 1, B)}, got {tuple(bnn.shape)}')
+
+    devs = {t.device for t in arrays if t.is_cuda}
+    if len(devs) > 1:
+        raise N.HflError(f'the octree tensors are on several devices: {sorted(map(str, devs))}')
+    if not torch.cuda.is_available():
+        raise N.HflError('the octree is imported on the GPU only (no CPU fallback)')
+    dev = devs.pop() if devs else torch.device('cuda', torch.cuda.current_device())
+    host = [j for j, t in enumerate(arrays) if not t.is_cuda]
+    if host:                                         # one pinned staging buffer -> one H2D copy
+        al = lambda x: (x + 255) // 256 * 256
+        sizes = [al(arrays[j].numel() * arrays[j].element_size()) for j in host]
+        stage = N.pinned.take(sum(sizes))
+        views, o = [], 0
+        for j, nb in zip(host, sizes):
+            t = arrays[j]
+            stage[o:o + nb].view(t.dtype)[:t.numel()].copy_(t.reshape(-1))
+            views.append((j, o, nb))
+            o += nb
+        devbuf = stage.to(dev, non_blocking=True)
+        N.pinned.mark()
+        for j, o, nb in views:
+            t = arrays[j]
+            arrays[j] = devbuf[o:o + nb].view(t.dtype)[:t.numel()].view(t.shape)
+    for d in range(D + 1):
+        desc.keys[d], desc.children[d] = arrays[d].data_ptr(), arrays[D + 1 + d].data_ptr()
+    desc.points = arrays[-1].data_ptr()
+
+    out = Octree(D, F, B, dev)
+    out._carve([B * 8 ** d if d <= F else nnum_nempty[d] for d in range(D + 1)], 0, n_status=2)
+    status = out._counts_dev[(D + 1) * (B + 2):]
+    ws_bytes = int(L.hfl_octree_import_workspace_bytes(C.byref(desc)))
+    ws = _arena(ws_bytes, dev)
+    with torch.cuda.device(dev):
+        N.check(L.hfl_octree_import(C.byref(desc), C.byref(out._desc), N.ptr(status), N.ptr(ws), ws_bytes,
+                                    N.stream()))
+        out._ocnn_batch_nnum_nempty = bnn.to(torch.int64)
+        out._read_back_counts()
+        out._pts_keepalive = (arrays, ws)
+        out._construct_ne_all()
+    return out
+
+
+def _check_import(status: torch.Tensor, batch_nnum_nempty: torch.Tensor, expected: torch.Tensor):
+    """Raise HflError for the invariants hfl_octree_import found violated, and for per-submap node
+    counts that disagree with the imported octree's batch_nnum_nempty."""
+    bits, depths = int(status[0]), int(status[1])
+    first = (depths & -depths).bit_length() - 1
+    if bits & N.HFL_IMPORT_BAD_CHILDREN:
+        raise N.HflError(f'ocnn octree import: invariant C (children) violated at depth {first}: the '
+                         f'non-negative children[d] must be 0, 1, ..., nnum_nempty[d]-1 in order')
+    if bits & N.HFL_IMPORT_BAD_KEYS:
+        raise N.HflError(f'ocnn octree import: invariant K (keys) violated at depth {first}: keys[d] must '
+                         f'be (submap << 48) | morton of the node, the parent key << 3 | child position')
+    bad = (batch_nnum_nempty != expected).any(1).nonzero()
+    if bad.numel():
+        d = int(bad[0])
+        raise N.HflError(f'ocnn octree import: batch_nnum_nempty[{d}] = {expected[d].tolist()} disagrees '
+                         f'with the per-submap node counts of the keys, {batch_nnum_nempty[d].tolist()}')
 
 
 def merge_octrees(octrees: Sequence[Octree]) -> Octree:

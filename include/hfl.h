@@ -74,6 +74,46 @@ size_t hfl_octree_build_workspace_bytes(int64_t n_points, int32_t batch, int32_t
 int hfl_octree_build(const float* points, const int32_t* pt_offsets, const hfl_octree* out,
                      void* workspace, size_t workspace_bytes, void* stream);
 
+/* An ocnn octree (SURVEY.md Appendix A) as the reference's collate_batch / to_device hand it to
+ * the model (eval/pnv_evaluate.py:122-126, 173-176).  Counts are host values; arrays are device
+ * arrays over ALL nodes of a depth:
+ *   keys[d]     [nnum[d]] int64 (submap << 48) | morton_d
+ *   children[d] [nnum[d]] int32 rank among the non-empty nodes of depth d, -1 if empty
+ *   points      [nnum_nempty[depth]*3] fp32 leaf means in octree units (ocnn points[depth]). */
+typedef struct hfl_ocnn_octree {
+  int32_t depth, full_depth, batch, _pad;
+  int64_t nnum[HFL_MAX_DEPTH + 1];
+  int64_t nnum_nempty[HFL_MAX_DEPTH + 1];
+  const int64_t* keys[HFL_MAX_DEPTH + 1];
+  const int32_t* children[HFL_MAX_DEPTH + 1];
+  const float* points;
+} hfl_ocnn_octree;
+
+/* Invariant bits of status[0] written by hfl_octree_import. */
+#define HFL_IMPORT_BAD_CHILDREN 1 /* non-negative children[d] are not 0,1,..,nnum_nempty[d]-1 in order */
+#define HFL_IMPORT_BAD_KEYS 2     /* keys[d] disagree with the node's position / its parent's key   */
+
+/* Host only, touches no device memory: the count relations hfl_octree_import checks first,
+ *   1 <= full_depth < depth <= 15, 1 <= batch < 32768, 0 <= nnum_nempty[d] <= nnum[d] < 2^31,
+ *   nnum[d] == batch*8^d (d <= full_depth), nnum_nempty[d] == nnum[d] (d < full_depth),
+ *   nnum[d] == 8*nnum_nempty[d-1] (d > full_depth).
+ * With them, every structural index of the import (such as the parent i >> 3 of node i) is in range. */
+int hfl_octree_import_check(const hfl_ocnn_octree* in);
+size_t hfl_octree_import_workspace_bytes(const hfl_ocnn_octree* in);
+
+/* Fills `out` (allocated for in->depth / full_depth / batch, cap[d] >= nnum_nempty[d] and
+ * cap[d] == batch*8^d for d <= full_depth) from an ocnn octree, so that it holds what
+ * hfl_octree_build writes for the same clouds: nkey, nidx, children, leaf_points and the counts
+ * table; point_leaf is not touched (ocnn does not keep it).  The host-side count relations are
+ * checked before any launch (HFL_ERR_INVALID).  The device-side invariants are checked by the
+ * kernels: status [2] int32 receives status[0] = HFL_IMPORT_* bits of the violated invariants and
+ * status[1] = a mask with bit d set for every depth d at which one failed.  Whatever the input,
+ * every index the output holds is in range, so the neighbour / token kernels may run on it; its
+ * values are meaningful only when status[0] == 0.  Lets HOTFormerLoc.forward
+ * (models/hotformerloc.py:33) take the ocnn octree the reference's callers build. */
+int hfl_octree_import(const hfl_ocnn_octree* in, const hfl_octree* out, int32_t* status,
+                      void* workspace, size_t workspace_bytes, void* stream);
+
 /* Replaces ocnn Octree.construct_neigh (misc/torch_utils.py:49-51).
  * Depth d <= full_depth: `grid` [batch*8^d*27] receives the full-grid table
  * (entries index ALL nodes), and na_out rows are gathered from it.
