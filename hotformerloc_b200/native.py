@@ -144,6 +144,10 @@ SIGNATURES = {
     'hfl_dwconv_inverse': (C.c_int, [_p, _i32, _i64, _i64, _i32, _p, _p]),
     'hfl_dwconv_wgrad_workspace_bytes': (C.c_int64, [_i64, _i32, _i32]),
     'hfl_dwconv_wgrad': (C.c_int, [_p, _p, _p, _i32, _i64, _i64, _i32, _i32, _p, _p, _i64, _p]),
+    'hfl_window_attn_train_fwd': (C.c_int, [_p, _p, _i32, _p, _i32, _p, _i64, _i32, _i32, _i32, _i32, _p, _p, _p]),
+    'hfl_window_attn_train_bwd_workspace_bytes': (C.c_int64, [_i32, _i32, _i32]),
+    'hfl_window_attn_train_bwd': (C.c_int, [_p, _p, _i32, _p, _i32, _p, _p, _p, _p, _i64, _i32, _i32, _i32, _i32,
+                                            _p, _p, _p, _i64, _p]),
 }
 
 

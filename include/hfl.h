@@ -300,6 +300,44 @@ int64_t hfl_dwconv_wgrad_workspace_bytes(int64_t n, int32_t K, int32_t C);
 int hfl_dwconv_wgrad(const float* grad, const float* data, const void* neigh, int32_t neigh_i64, int64_t n,
                      int64_t n_in, int32_t K, int32_t C, float* dw, void* ws, int64_t ws_bytes, void* stream);
 
+/* ------------------------------------------------------------------------
+ * Octree window attention core with backward, fp32 (training side, not called by the embedding
+ * path): OctreeAttention.forward from qkv to before proj, with the RPE bias, the submap mask and
+ * the H-OSA relay token.  For window n, head h (head dim 16, C = 16 H, 1 <= H <= 16), queries i and
+ * keys j of the L = K + hat window positions (1 <= L <= 128):
+ *   s = (q_i . k_j) 0.25 + (ids[n,i] == ids[n,j] ? 0 : -1000)
+ *       + sum_a rpe_table[clamp(x_ia - x_ja, -bnd, bnd) + bnd + a (2 bnd + 1), h]
+ *   o[n,i,16h+e] = sum_j softmax_j(s) v[n,h,j,e]
+ * With hat = 1 the relay token is position 0 and its row and column get no RPE term.
+ *   qkv  [n_win, L, 3C] fp32, the output of Linear(C, 3C): column of (s, h, e) = s C + 16 h + e
+ *   xyz  [n_win, L - hat, 3] int32 / int64 (xyz_i64) integer cell coordinates of the window tokens
+ *        (after any dilation gather); may be NULL when rpe_table is NULL
+ *   ids  [n_win, L] int32 / int64 (ids_i64); tokens attend with bias 0 iff their ids are equal
+ *   rpe_table [3 (2 bnd + 1), H] fp32 or NULL (no RPE), 0 <= bnd <= 2^20
+ *   o    [n_win, L, C] fp32, lse [n_win, H, L] fp32 (per-row log-sum-exp, kept for the backward)
+ * qkv, o, dout and dqkv must be 16-byte aligned.  No [n_win, H, L, L] tensor is written.
+ * ------------------------------------------------------------------------ */
+
+/* Replaces OctreeAttention.forward's core (octformer_backbone.py:52-93), the RPE gather
+ * (octformer_layers.py:156-170) and HOTFormerBlock's relay-token attention (hotformerloc_backbone.py:197-236). */
+int hfl_window_attn_train_fwd(const float* qkv, const void* xyz, int32_t xyz_i64, const void* ids, int32_t ids_i64,
+                              const float* rpe_table, int64_t n_win, int32_t L, int32_t H, int32_t hat, int32_t bnd,
+                              float* o, float* lse, void* stream);
+
+/* Backward of hfl_window_attn_train_fwd (octformer_backbone.py:52-93, octformer_layers.py:156-170,
+ * hotformerloc_backbone.py:197-236 under autograd): given dout [n_win, L, C] and the forward's o and
+ * lse, writes dqkv [n_win, L, 3C] and, with a table, drpe_table [3 (2 bnd + 1), H] (three bins per
+ * token pair, nothing from the relay token's row or column).  Every dqkv element is a fixed-order
+ * fp32 sum; the table gradient is summed in exact int64 fixed point (range argument in
+ * csrc/window_attn_train.cu).  Both are bit-identical across runs, without float atomics.
+ * ws: hfl_window_attn_train_bwd_workspace_bytes(H, bnd, rpe_table != NULL) bytes, 256-byte aligned
+ * (0 bytes and NULL without a table). */
+int64_t hfl_window_attn_train_bwd_workspace_bytes(int32_t H, int32_t bnd, int32_t has_rpe);
+int hfl_window_attn_train_bwd(const float* qkv, const void* xyz, int32_t xyz_i64, const void* ids, int32_t ids_i64,
+                              const float* rpe_table, const float* o, const float* lse, const float* dout,
+                              int64_t n_win, int32_t L, int32_t H, int32_t hat, int32_t bnd, float* dqkv,
+                              float* drpe_table, void* ws, int64_t ws_bytes, void* stream);
+
 /* Exact L2 top-k (eval/pnv_evaluate.py:200-225, 245) on one database shard, and the
  * merge of all-gathered partial lists. */
 int hfl_knn_topk(const float* q, int32_t nq, const float* db, int32_t ndb, int32_t dim, int32_t k,
