@@ -148,6 +148,10 @@ SIGNATURES = {
     'hfl_window_attn_train_bwd_workspace_bytes': (C.c_int64, [_i32, _i32, _i32]),
     'hfl_window_attn_train_bwd': (C.c_int, [_p, _p, _i32, _p, _i32, _p, _p, _p, _p, _i64, _i32, _i32, _i32, _i32,
                                             _p, _p, _p, _i64, _p]),
+    'hfl_attn_pool_train_fwd_workspace_bytes': (C.c_int64, [_i64, _i32, _i32, _i32]),
+    'hfl_attn_pool_train_bwd_workspace_bytes': (C.c_int64, [_i64, _i32, _i32, _i32]),
+    'hfl_attn_pool_train_fwd': (C.c_int, [_p, _p, _p, _i64, _i32, _i32, _i32, _p, _p, _p, _i64, _p]),
+    'hfl_attn_pool_train_bwd': (C.c_int, [_p, _p, _p, _p, _p, _p, _i64, _i32, _i32, _i32, _p, _p, _p, _i64, _p]),
 }
 
 

@@ -338,6 +338,41 @@ int hfl_window_attn_train_bwd(const float* qkv, const void* xyz, int32_t xyz_i64
                               int64_t n_win, int32_t L, int32_t H, int32_t hat, int32_t bnd, float* dqkv,
                               float* drpe_table, void* ws, int64_t ws_bytes, void* stream);
 
+/* ------------------------------------------------------------------------
+ * Attention pooling over ragged per-submap token segments with backward, fp32 (training side, not
+ * called by the embedding path): the AdaptivePooling of PyramidAttnPoolWrapper without the padded
+ * (B, Nmax, C) features and the (B, N, N) mask.  Segment b = tokens [offsets[b], offsets[b+1]) of
+ * x [n, C]; queries Q [k, C]; s = C^-0.5:
+ *   S[b,q,t] = s Q[q].x[t]     out[b,q] = sum_t softmax_t(S[b,q,.]) x[t]     lse[b,q] = log sum_t exp(S[b,q,t])
+ * An empty segment gives out = 0 and lse = -inf, and contributes no gradient.
+ *   offsets [B+1] int64 (device); each entry is clamped into [0, n] and a decreasing pair is an empty
+ *           segment, so no offsets value makes a kernel access memory out of range.  The results are
+ *           those of the formula when the offsets are non-decreasing with offsets[0] = 0 and
+ *           offsets[B] = n (every token in exactly one segment).
+ *   1 <= k <= 256, C a multiple of 32 in [32, 512], n >= 0, 1 <= B <= 2^24;
+ *   x, Q, dout 16-byte aligned; out, dout [B, k, C]; lse [B, k]; dx [n, C]; dQ [k, C].
+ * Tokens are cut into segment-aligned chunks of 1024; the partition depends on (offsets, k, C) only
+ * and every output element is a fixed-order fp32 sum (no float atomics, no TF32): out, lse, dx and dQ
+ * are bit-identical across runs.  Workspaces: the *_workspace_bytes of (n, B, k, C), 256-byte
+ * aligned, (ceil(n / 1024) + B) k (C + 2) 4 bytes forward and (ceil(n / 1024) + B) k C 4 bytes
+ * backward, plus O(B k).
+ * ------------------------------------------------------------------------ */
+int64_t hfl_attn_pool_train_fwd_workspace_bytes(int64_t n, int32_t B, int32_t k, int32_t C);
+int64_t hfl_attn_pool_train_bwd_workspace_bytes(int64_t n, int32_t B, int32_t k, int32_t C);
+
+/* Replaces the split / pad of the local features to (B, Nmax, C), the (B, N, N) int64 mask and the
+ * single-head attention of the learned queries (models/layers/pooling.py:183-233, salsa.py:25-55). */
+int hfl_attn_pool_train_fwd(const float* x, const int64_t* offsets, const float* Q, int64_t n, int32_t B, int32_t k,
+                            int32_t C, float* out, float* lse, void* ws, int64_t ws_bytes, void* stream);
+
+/* Backward of hfl_attn_pool_train_fwd (pooling.py:183-233, salsa.py:25-55 under autograd): given dout
+ * and the forward's out and lse, writes dx = sum_q p dout[b,q] + s sum_q dS Q[q] and
+ * dQ = s sum_t dS x[t], with dS = p (dout[b,q].x[t] - dout[b,q].out[b,q]) and p recomputed from x, Q
+ * and lse. */
+int hfl_attn_pool_train_bwd(const float* x, const int64_t* offsets, const float* Q, const float* out,
+                            const float* lse, const float* dout, int64_t n, int32_t B, int32_t k, int32_t C,
+                            float* dx, float* dQ, void* ws, int64_t ws_bytes, void* stream);
+
 /* Exact L2 top-k (eval/pnv_evaluate.py:200-225, 245) on one database shard, and the
  * merge of all-gathered partial lists. */
 int hfl_knn_topk(const float* q, int32_t nq, const float* db, int32_t ndb, int32_t dim, int32_t k,
