@@ -14,7 +14,7 @@ models/layers/pooling.py:183-233.
 """
 from __future__ import annotations
 
-from typing import Dict, List, Optional, Sequence
+from typing import Dict, List, NamedTuple, Optional, Sequence
 
 import numpy as np
 import torch
@@ -334,6 +334,50 @@ def _f(t):
 
 def _conv_w(conv: _OctConv):
     return _bf(conv.weights.detach().flatten(0, 1).t())          # [Cout, kdim*Cin]
+
+
+class RTOwnership(NamedTuple):
+    """Relay-token sequences of a pyramid; see :func:`rt_ownership`."""
+    num_windows: List[np.ndarray]     # per level: (B,) int64 windows (RTs) owned by each submap
+    pos: List[np.ndarray]             # per level: (N_win_j,) int64 packed row of each window
+    ids: np.ndarray                   # (T,) int64 attention id of each packed row
+    cu: np.ndarray                    # (B + 1,) int64 sequence offsets
+    total: int                        # T, all windows of all levels
+    max_len: int                      # longest sequence
+
+
+def rt_ownership(level_counts: Sequence[np.ndarray], patch_size: int, n_pad: Sequence[int]) -> RTOwnership:
+    """Which submap's relay-token sequence each window of each pyramid level joins, and where
+    (models/octree.py:156-184, 229-265; relay_token_utils.py:12-40), from the host per-submap node
+    counts of each level, fine to coarse, and each level's padded token count n_pad[j] (OctreeT pads to a
+    multiple of patch_size * dilation).
+
+    Level j's n_pad[j] tokens are cut into windows of patch_size tokens.  A window belongs to the
+    submap of its first token, and the windows that hold only padding belong to the last submap.  Submap b's sequence is its windows of level 0, then of
+    level 1, ..., each in window order; the sequences are packed back to back in submap order.  A
+    row's id is its submap, or B for a window that holds only padding (its RT never attends to a
+    real one).  Shared by the inference engine's tables and the training-side layout."""
+    K = patch_size
+    counts = [np.asarray(c, dtype=np.int64) for c in level_counts]
+    B = counts[0].size
+    nws = []
+    for c, npad in zip(counts, n_pad):
+        cum = np.cumsum(c)
+        cum[-1] += int(npad) - int(c.sum())             # the padding tokens follow the last submap's
+        nws.append(np.diff(np.concatenate([[0], -(-cum // K)])))
+    tot = np.sum(nws, axis=0)
+    cu = np.concatenate([[0], np.cumsum(tot)]).astype(np.int64)
+    ids = np.empty(int(cu[-1]), dtype=np.int64)
+    pos, prefix = [], np.zeros(B, dtype=np.int64)
+    for c, nw in zip(counts, nws):
+        wi = np.arange(int(nw.sum()), dtype=np.int64)
+        owner = np.repeat(np.arange(B, dtype=np.int64), nw)
+        start = np.cumsum(nw) - nw
+        p = cu[owner] + prefix[owner] + (wi - start[owner])
+        ids[p] = np.where(wi >= -(-int(c.sum()) // K), B, owner)   # windows from here on hold only padding
+        pos.append(p)
+        prefix += nw
+    return RTOwnership(nws, pos, ids, cu, int(cu[-1]), int(tot.max()))
 
 
 class _Engine:
@@ -695,34 +739,24 @@ class _Engine:
             ops.gem_head(pooled, gw['w'], g, b, mu, var, eps, self.normalize_embeddings, out)
         return out
 
+    @staticmethod
+    def _rt_tables(counts, npad, nwin, R, K):
+        """The RT sequences of the pyramid (rt_ownership) and each packed row's row in the hat layout:
+        window wi of level j sits at R[j] + wi (K + 1)."""
+        own = rt_ownership(counts, K, npad)
+        rt_rows = np.empty(own.total, dtype=np.int32)
+        for j in range(len(counts)):
+            rt_rows[own.pos[j]] = R[j] + np.arange(nwin[j], dtype=np.int64) * (K + 1)
+        return own, rt_rows
+
     def _host_tables(self, octree, depths, nl, npad, nwin, R, K, B):
         """Relay-token ownership / sequence tables (models/octree.py:156-184, 229-265;
         relay_token_utils.py:12-40) from the host copy of the node counts; one
         pinned staging buffer, one H2D copy."""
         L = len(depths)
         counts = [octree.batch_nnum_nempty[dj].numpy().astype(np.int64) for dj in depths]
-        nws, starts = [], []
-        for j in range(L):
-            cum = np.cumsum(counts[j])
-            cum[-1] += npad[j] - nl[j]
-            boundary = -(-cum // K)
-            nw = np.diff(np.concatenate([[0], boundary]))
-            nws.append(nw)
-            starts.append(np.cumsum(nw) - nw)
-        tot = np.sum(nws, axis=0)
-        cu = np.concatenate([[0], np.cumsum(tot)]).astype(np.int32)
-        total_rt = int(cu[-1])
-        rt_rows = np.empty(total_rt, dtype=np.int32)
-        ids = np.empty(total_rt, dtype=np.int32)
-        prefix = np.zeros(B, dtype=np.int64)
-        for j in range(L):
-            wi = np.arange(nwin[j], dtype=np.int64)
-            owner = np.repeat(np.arange(B, dtype=np.int64), nws[j])
-            pos = cu[owner] + prefix[owner] + (wi - starts[j][owner])
-            rt_rows[pos] = R[j] + wi * (K + 1)
-            first_pad = -(-nl[j] // K)                  # windows >= this hold only padding
-            ids[pos] = np.where(wi >= first_pad, B, owner)
-            prefix += nws[j]
+        own, rt_rows = self._rt_tables(counts, npad, nwin, R, K)
+        nws, cu, ids, total_rt = own.num_windows, own.cu.astype(np.int32), own.ids.astype(np.int32), own.total
         tok_off = [np.concatenate([[0], np.cumsum(c)]).astype(np.int32) for c in counts]
         rt_local = [(np.arange(nwin[j], dtype=np.int64) * (K + 1)).astype(np.int32) for j in range(L)]
         parts = [rt_rows, ids, cu] + tok_off + rt_local
@@ -740,7 +774,7 @@ class _Engine:
             o += s
         return dict(rt_rows=views[0], ids=views[1], cu=views[2], tok_off=views[3:3 + L],
                     rt_local=views[3 + L:3 + 2 * L], total_rt=total_rt,
-                    max_len=int(tot.max()), num_windows=nws)
+                    max_len=own.max_len, num_windows=nws)
 
 
 class HOTFormerLoc(nn.Module):

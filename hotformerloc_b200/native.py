@@ -152,6 +152,9 @@ SIGNATURES = {
     'hfl_attn_pool_train_bwd_workspace_bytes': (C.c_int64, [_i64, _i32, _i32, _i32]),
     'hfl_attn_pool_train_fwd': (C.c_int, [_p, _p, _p, _i64, _i32, _i32, _i32, _p, _p, _p, _i64, _p]),
     'hfl_attn_pool_train_bwd': (C.c_int, [_p, _p, _p, _p, _p, _p, _i64, _i32, _i32, _i32, _p, _p, _p, _i64, _p]),
+    'hfl_rt_attn_train_workspace_bytes': (C.c_int64, [_i64, _i32, _i32]),
+    'hfl_rt_attn_train_fwd': (C.c_int, [_p, _p, _p, _i32, _i32, _i64, _i32, _p, _p, _p, _i64, _p]),
+    'hfl_rt_attn_train_bwd': (C.c_int, [_p, _p, _p, _i32, _p, _p, _p, _i32, _i64, _i32, _p, _p, _i64, _p]),
 }
 
 

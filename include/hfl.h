@@ -373,6 +373,42 @@ int hfl_attn_pool_train_bwd(const float* x, const int64_t* offsets, const float*
                             const float* lse, const float* dout, int64_t n, int32_t B, int32_t k, int32_t C,
                             float* dx, float* dQ, void* ws, int64_t ws_bytes, void* stream);
 
+/* ------------------------------------------------------------------------
+ * Relay-token self-attention core with backward, fp32 (training side, not called by the embedding
+ * path): RTAttention.forward from qkv to before proj over the ragged per-submap RT sequences, without
+ * concat_and_pad_rt's (B, Nmax, C) tensors and the (B, Nmax, Nmax) mask.  Sequence b = packed rows
+ * [cu[b], cu[b+1]) of T; for head h (head dim 16, C = 16 H, 1 <= H <= 16) and rows i, j of one sequence:
+ *   s_ij = 0.25 q_i.k_j + (ids[i] == ids[j] ? 0 : -1000)
+ *   o[i, 16h+e] = sum_j softmax_j(s_i.) v_j[e]          lse[i, h] = log sum_j exp(s_ij)
+ * The reference's padding slots carry -1000 against every real RT, so their weight is exactly 0 in
+ * fp32 and the ragged form equals the padded one at every real row.
+ *   qkv [T, 3C] fp32, the output of Linear(C, 3C): column of (s, h, e) = s C + 16 h + e
+ *   cu  [B+1] int32 (device); each entry is clamped into [0, T] and never below the previous entry's
+ *       clamped value, so a decreasing pair is an empty sequence, an entry above T cuts its sequence at
+ *       T, sequences never overlap, and no cu value makes a kernel access memory out of range.  Rows in
+ *       no sequence are not written.  A sequence may have any length from 0 to T.
+ *   ids [T] int32 / int64 (ids_i64); rows attend with bias 0 iff their ids are equal (any values)
+ *   o [T, C], lse [T, H], dout [T, C], dqkv [T, 3C] fp32; qkv, o, dout and dqkv 16-byte aligned
+ *   1 <= B <= 2^24, T >= 0 with 3 C T < 2^31
+ * Every output element is a fixed-order fp32 sum (no float atomics, no TF32): o, lse and dqkv are
+ * bit-identical across runs.  ws: hfl_rt_attn_train_workspace_bytes(T, B, H) bytes, 256-byte aligned
+ * (2 (B + 1) + T H 4-byte words, rounded up), for the forward and the backward alike.
+ * ------------------------------------------------------------------------ */
+int64_t hfl_rt_attn_train_workspace_bytes(int64_t T, int32_t B, int32_t H);
+
+/* Replaces RTAttention.forward's core (hotformerloc_backbone.py:83-119) with the mask of
+ * models/octree.py:229-265, and the padding of concat_and_pad_rt (relay_token_utils.py:12-40). */
+int hfl_rt_attn_train_fwd(const float* qkv, const int32_t* cu, const void* ids, int32_t ids_i64, int32_t B,
+                          int64_t T, int32_t H, float* o, float* lse, void* ws, int64_t ws_bytes, void* stream);
+
+/* Backward of hfl_rt_attn_train_fwd (hotformerloc_backbone.py:83-119 under autograd): given dout and the
+ * forward's o and lse, writes dqkv: with D_i = dO_i.o_i and p = exp(s - lse) recomputed from qkv,
+ * dq_i = 0.25 sum_j p_ij (dO_i.v_j - D_i) k_j by query rows, then dk_j = 0.25 sum_i dS_ij q_i and
+ * dv_j = sum_i p_ij dO_i by key rows over the queries of the key's own sequence. */
+int hfl_rt_attn_train_bwd(const float* qkv, const int32_t* cu, const void* ids, int32_t ids_i64, const float* o,
+                          const float* lse, const float* dout, int32_t B, int64_t T, int32_t H, float* dqkv, void* ws,
+                          int64_t ws_bytes, void* stream);
+
 /* Exact L2 top-k (eval/pnv_evaluate.py:200-225, 245) on one database shard, and the
  * merge of all-gathered partial lists. */
 int hfl_knn_topk(const float* q, int32_t nq, const float* db, int32_t ndb, int32_t dim, int32_t k,
