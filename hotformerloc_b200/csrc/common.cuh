@@ -31,12 +31,14 @@ inline int fail(int code, const char* fmt, const char* a = "", long long b = 0) 
                          cudaGetErrorString(e__), (long long)__LINE__);       \
   } while (0)
 
-// kernel<<<...>>> launch + bookkeeping + error peek (no sync)
+// kernel<<<...>>> launch + bookkeeping + launch-error check (no sync).  cudaGetLastError clears the
+// error it reports, so a rejected launch (e.g. a bad configuration) fails this call only and not every later
+// call of the thread; a sticky device fault stays visible to everyone whatever we do here.
 #define HFL_LAUNCH(...)                                                       \
   do {                                                                        \
     __VA_ARGS__;                                                              \
     ::hfl::g_launches.fetch_add(1, std::memory_order_relaxed);                \
-    HFL_CUDA(cudaPeekAtLastError());                                          \
+    HFL_CUDA(cudaGetLastError());                                             \
   } while (0)
 
 // cudaFuncAttributeMaxDynamicSharedMemorySize is per device: remember the largest size requested per

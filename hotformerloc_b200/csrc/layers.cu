@@ -767,6 +767,7 @@ int hfl_attn_pool(const float* logits, const float* x, const void* xb, const int
                   float* stat, float* out, int32_t B, int32_t kq, int32_t ldl, int32_t K, int32_t C,
                   int32_t ktot, int32_t q_off, float scale, void* stream_) {
   cudaStream_t st = (cudaStream_t)stream_;
+  if (B == 0 || kq == 0) return HFL_OK;     // empty problem: no zero-sized grid
   HFL_CHECK_ARG(logits && xb && tok_off && stat && out, "null argument");
   HFL_CHECK_ARG(C == 256, "C must be 256");
   PoolParams p{logits, x, (const __nv_bfloat16*)xb, tok_off, stat, out, B, kq, ldl, K, C, ktot, q_off, scale};
@@ -780,6 +781,7 @@ int hfl_mixer_tail(const float* x, const float* wc, const float* bc, const float
                    const float* br, float* out, int32_t B, int32_t kin, int32_t kout, int32_t C,
                    int32_t od, int32_t normalize, void* stream_) {
   cudaStream_t st = (cudaStream_t)stream_;
+  if (B == 0) return HFL_OK;
   HFL_CHECK_ARG(x && wc && bc && wr && br && out, "null argument");
   HFL_CHECK_ARG(C == 256 || C == 128, "C must equal the CTA size (128/256)");
   TailParams p{x, wc, bc, wr, br, out, kin, kout, C, od, normalize};
@@ -791,6 +793,7 @@ int hfl_mixer_tail(const float* x, const float* wc, const float* bc, const float
 
 int hfl_gem_pool(const float* x, const int32_t* tok_off, int32_t B, int32_t K, int32_t C, float pw,
                  float eps, float* out, int32_t ld_out, int32_t col_off, void* stream_) {
+  if (B == 0) return HFL_OK;
   HFL_CHECK_ARG(x && tok_off && out, "null argument");
   HFL_LAUNCH((k_gem_pool<<<B, 256, 0, (cudaStream_t)stream_>>>(x, tok_off, K, C, pw, eps, out, ld_out, col_off)));
   return HFL_OK;
@@ -799,6 +802,7 @@ int hfl_gem_pool(const float* x, const int32_t* tok_off, int32_t B, int32_t K, i
 int hfl_gem_head(const float* pooled, int32_t B, int32_t in_dim, const float* w, const float* bn_g,
                  const float* bn_b, const float* bn_mean, const float* bn_var, float bn_eps,
                  int32_t out_dim, int32_t normalize, float* out, void* stream_) {
+  if (B == 0) return HFL_OK;
   HFL_CHECK_ARG(pooled && w && bn_g && bn_b && bn_mean && bn_var && out, "null argument");
   HFL_CHECK_ARG(out_dim <= 1024 && in_dim * 4 <= 48 * 1024, "head too large");
   HFL_LAUNCH((k_gem_head<<<B, 256, in_dim * 4, (cudaStream_t)stream_>>>(pooled, in_dim, w, bn_g, bn_b, bn_mean, bn_var, bn_eps, out_dim, normalize, out)));
