@@ -409,6 +409,36 @@ int hfl_rt_attn_train_bwd(const float* qkv, const int32_t* cu, const void* ids, 
                           const float* lse, const float* dout, int32_t B, int64_t T, int32_t H, float* dqkv, void* ws,
                           int64_t ws_bytes, void* stream);
 
+/* ------------------------------------------------------------------------
+ * Octree convolution with backward, fp32 without TF32 (training side, not called by the embedding path):
+ * ocnn.nn.OctreeConv for kernel 333 / stride 1 and kernel 222 / stride 2, nempty.
+ *   neigh [n_out, K] int32 / int64 (neigh_i64), K in {8, 27}; an entry outside [0, n_in) is an empty tap
+ *   data [n_in, Cin], w [K, Cin, Cout] (ocnn's `weights`), out [n_out, Cout]; 1 <= Cin, Cout <= 256
+ * Work follows the occupied (row, tap) pairs: per tile of 128 output rows and tap the rows holding the
+ * tap are compacted on the device before the tap's product runs.  Every output element is a fixed-order
+ * fp32 sum (no float atomics): results are bit-identical across runs, GPUs and table dtypes.  The
+ * rounding chains are documented in csrc/octree_conv_train.cu.
+ * ------------------------------------------------------------------------ */
+
+/* out[i,:] = sum_k sum_c data[neigh[i,k],c] w[k,c,:] over the occupied taps.  With the inverse table
+ * (hfl_dwconv_inverse over neigh with n_data = n_in: stride 1 inv[j,k] = i where neigh[i,k] = j; stride 2
+ * each input row's parent at its child position), the per-tap transposed weights [K, Cout, Cin] and the
+ * output gradient in place of data it is the input gradient.
+ * Replaces ocnn.nn.OctreeConv (octformer_layers.py:80-98 / :89, octformer_backbone.py:451-477 / :470). */
+int hfl_octree_conv_train_fwd(const float* data, const void* neigh, int32_t neigh_i64, const float* w, int64_t n_out,
+                              int64_t n_in, int32_t K, int32_t Cin, int32_t Cout, float* out, void* stream);
+
+/* dw[k] = sum_i data[neigh[i,k]]^T (x) dout[i] over the occupied pairs; dout [n, Cout], dw [K, Cin, Cout].
+ * Rows are cut into chunks that depend on (n, K, Cin, Cout) only; per-chunk partials go to ws and are
+ * folded in chunk order.  ws: hfl_octree_conv_train_wgrad_workspace_bytes(n, K, Cin, Cout) bytes, 16-byte
+ * aligned (at most 128 MiB).  n = 0 writes zeros.
+ * Replaces the weight gradient of ocnn.nn.OctreeConv (octformer_layers.py:80-98 / :89,
+ * octformer_backbone.py:451-477 / :470) under autograd. */
+int64_t hfl_octree_conv_train_wgrad_workspace_bytes(int64_t n, int32_t K, int32_t Cin, int32_t Cout);
+int hfl_octree_conv_train_wgrad(const float* data, const void* neigh, int32_t neigh_i64, const float* dout, int64_t n,
+                                int64_t n_in, int32_t K, int32_t Cin, int32_t Cout, float* dw, void* ws,
+                                int64_t ws_bytes, void* stream);
+
 /* Exact L2 top-k (eval/pnv_evaluate.py:200-225, 245) on one database shard, and the
  * merge of all-gathered partial lists. */
 int hfl_knn_topk(const float* q, int32_t nq, const float* db, int32_t ndb, int32_t dim, int32_t k,
