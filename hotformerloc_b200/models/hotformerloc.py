@@ -208,6 +208,11 @@ class HOTFormer(nn.Module):
             if isinstance(m, nn.Linear):
                 _trunc(m.weight)
                 nn.init.zeros_(m.bias)
+        self.drop_path = drop_path
+        self.grad_checkpoint = grad_checkpoint
+        # True: forward runs the differentiable fp32 graph (models/differentiable.py) instead of the bf16
+        # inference engine.  A plain attribute, not a parameter or buffer: the state_dict is unchanged.
+        self.differentiable = False
         self._own_engine = None
 
     def forward(self, data, octree: Octree, depth: int):
@@ -216,7 +221,17 @@ class HOTFormer(nn.Module):
         ``data`` must be ``InputFeature('P', nempty=True)(octree)`` -- the leaf point means the first
         kernel reads straight from the octree (only input_features='P' is on the hot path): it is
         checked for shape and otherwise not re-read.  ``octree`` may be an ocnn octree; the third
-        output is then the native Octree imported from it."""
+        output is then the native Octree imported from it.
+
+        With ``differentiable`` set, the outputs come from the fp32 training kernels with autograd and
+        ``data`` is the stem's input, so it receives a gradient if it requires one."""
+        if self.differentiable:
+            from .differentiable import backbone_forward, check_trainable   # imports this module
+            check_trainable(self)
+            octree = _native_octree(octree)
+            assert depth == octree.depth, 'the backbone starts at the leaf depth of the octree'
+            local, relay = backbone_forward(self, data, octree)
+            return local, relay, octree
         octree = _native_octree(octree)
         assert depth == octree.depth, 'the backbone starts at the leaf depth of the octree'
         if data is not None:
@@ -802,7 +817,20 @@ class HOTFormerLoc(nn.Module):
         """Re-read the parameters on the next forward (needed only after writes through ``.data``)."""
         self._engine.invalidate()
 
+    @property
+    def differentiable(self) -> bool:
+        """Whether ``forward`` runs the differentiable fp32 graph (models/differentiable.py) rather than the bf16
+        inference engine; reads and writes ``backbone.differentiable``.  Default False."""
+        return self.backbone.differentiable
+
+    @differentiable.setter
+    def differentiable(self, value: bool):
+        self.backbone.differentiable = bool(value)
+
     def forward(self, batch):
+        if self.differentiable:
+            from .differentiable import model_forward        # imports this module
+            return {'global': model_forward(self, batch['octree'])}
         octree = _native_octree(batch['octree'])
         self._engine.normalize_embeddings = self.normalize_embeddings
         x = self._engine.forward(octree)

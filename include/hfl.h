@@ -439,6 +439,29 @@ int hfl_octree_conv_train_wgrad(const float* data, const void* neigh, int32_t ne
                                 int64_t n_in, int32_t K, int32_t Cin, int32_t Cout, float* dw, void* ws,
                                 int64_t ws_bytes, void* stream);
 
+/* ------------------------------------------------------------------------
+ * Relay-token initialisation with backward, fp32 (training side, not called by the embedding path):
+ * RelayTokenInitialiser.forward (hotformerloc_backbone.py:345-363) and the ADaPE window statistics of
+ * OctreeT.compute_window_stats (models/octree.py:285-344).  Window w = rows [w K, (w + 1) K) of
+ *   xyzb [n_win K, 4] int16 (x, y, z, submap), Octree.tokens(depth, n_win K): padding rows are (0, 0, 0, B)
+ *   src  [n, C] fp32, the level's tokens; rows n <= t < n_win K are padding and count as zeros
+ * A row is valid when its submap equals the window's first row's; cnt = number of valid rows (>= 1).
+ *   rt_out [n_win, C]:  rt[w] = (sum of src over the valid rows) / cnt  (0 for an all-padding window)
+ *   stats_out [n_win, mode] with mode 3 'pos' | 6 'var' | 9 'cov' (0: none, stats_out unused): the mean of
+ *     the node centres xyz 2^(1-depth) - 1 (set to 0 at padding rows after the rescale) over max(cnt, 1),
+ *     then the variances ('var') or upper-triangle covariances xx xy xz yy yz zz ('cov') with Bessel's
+ *     correction max(cnt - 1, 1), zeroed unless cnt >= 2.  The statistics carry no gradient.
+ * C a multiple of 32 in [32, 512]; 1 <= K <= 4096; 0 <= n <= n_win K; xyzb 8-byte aligned.
+ * Fixed-order sums, no atomics: bit-identical across runs.
+ * ------------------------------------------------------------------------ */
+int hfl_rt_init_train_fwd(const float* src, const int16_t* xyzb, int64_t n, int64_t n_win, int32_t K, int32_t C,
+                          int32_t depth, int32_t mode, float* rt_out, float* stats_out, void* stream);
+
+/* Backward of hfl_rt_init_train_fwd: grad_src [n, C], grad_src[t] = grad_rt[w(t)] / cnt[w(t)] at the valid
+ * rows and 0 at the others.  Each row lies in exactly one window, so it is a gather. */
+int hfl_rt_init_train_bwd(const float* grad_rt, const int16_t* xyzb, int64_t n, int64_t n_win, int32_t K, int32_t C,
+                          float* grad_src, void* stream);
+
 /* Exact L2 top-k (eval/pnv_evaluate.py:200-225, 245) on one database shard, and the
  * merge of all-gathered partial lists. */
 int hfl_knn_topk(const float* q, int32_t nq, const float* db, int32_t ndb, int32_t dim, int32_t k,
